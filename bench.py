@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (libdfk.so)
   python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port, all host threads)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
 
 Workload (BASELINE.json configs[1]): one evaluation = SfmAligner::RunStep over the 4-level pyramid
 (640x480 ... 80x60, 408 000 px) of one keyframe/frame pair at code size 32, synthetic data
@@ -31,6 +32,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 
 METRIC = "keyframe-pair Jacobian+JtJ evals/sec (640x480, C=32)"
 W0, H0, CS, LEVELS = 640, 480, 32, 4
@@ -68,7 +70,14 @@ def parse():
     ap.add_argument("--sustain-seconds", type=float, default=1.2,
                     help="after the K timed steps, repeat the same step back to back for about this long (clocks are sampled "
                          "over both regions); reported as `sustained`")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (per work item: "
+                         "JtJ packed upper, Jtr, residual, inliers; the window's block-sparse buffer), for comparing two "
+                         "builds on the same seeded inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -285,8 +294,7 @@ def run_reference_arm(args):
         sweep_res[c] = v
         if v > best_v:
             best_t, best_v = c, v
-    t_step = best_t / best_v
-    steps = max(1, min(max(1, args.steps), max(3, int(150.0 / max(t_step, 1e-3)))))
+    steps = max(1, args.steps)
     dt = run(best_t, steps)
     val = best_t * steps / dt
     out = {"impl": "reference", "metric": METRIC, "value": val, "unit": "evals/s", "n_gpus": args.gpus,
@@ -432,6 +440,29 @@ def window_pairs(num_kf: int, num_pairs: int, seed: int = 2):
             seen.add((a, b))
             pairs.append((a, b))
     return pairs
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, cs, records, window):
+    """--dump-outputs: the result records of one step and the window buffer they were assembled into, as float32 / float64
+    .npy files.  Above DUMP_BYTES in all, every array is flattened and keeps the same share of its elements, at positions
+    drawn from a fixed seed, so two runs of one configuration store the same positions."""
+    import numpy as np
+
+    from deepfactors_b200 import factors
+    n, nh, _ = factors.record_layout(cs)
+    arrays = {"JtJ": records[:, :nh], "Jtr": records[:, nh:nh + n], "residual": records[:, nh + n],
+              "inliers": np.ascontiguousarray(records[:, nh + n + 1]).view(np.uint32).astype(np.float64),
+              "window": window}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.size * (DUMP_BYTES - (1 << 16)) // total   # headroom for the .npy headers
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a))
 
 
 def main():
@@ -613,6 +644,8 @@ def main():
     drain_comm()                      # the last steps' all-reduces belong to the timed region
     e1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cs, records.cpu().numpy(), wbuf[(step_no[0] - 1) & 1].cpu().numpy())
     if world > 1:
         dist.barrier()
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
